@@ -40,7 +40,10 @@ KEY_SALT = 0x9E3779B97F4A7C15
 def parse_args():
   ap = argparse.ArgumentParser()
   ap.add_argument("--gpus", type=int, default=1)
-  ap.add_argument("--steps", type=int, default=2000)
+  ap.add_argument("--steps", type=int, default=2000,
+                  help="timed steps of every GPU measurement: the headline and the c3 line (embedded or --workload c3); "
+                       "the CPU arms time a bounded sample of their own (--impl reference: 20-40 steps, the embedded "
+                       "cpu_baseline: 15), reported as their own `steps`")
   ap.add_argument("--warmup", type=int, default=20)
   ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
   ap.add_argument("--resident", type=int, default=100_000_000, help="resident keys per GPU")
@@ -66,7 +69,12 @@ def parse_args():
                   help="c3 / c5: per-unique gradient sum by det_segment_reduce (position order, deterministic) or by "
                        "torch index_add (atomics); sets DET_GRAD_REDUCE for the sharded combine as well")
   ap.add_argument("--distinct-batches", type=int, default=64, help="distinct key batches cycled through")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="after the timed steps, write a fixed sample of the rows the last timed step returned as "
+                       "DIR/<name>.npy (float32): lookup_rows (c2 / c4) and c3_lookup_sparse (c3, also embedded in c2)")
   a = ap.parse_args()
+  if a.dump_outputs and (a.impl == "reference" or a.workload == "c5"):
+    ap.error("--dump-outputs covers the c2, c3 and c4 workloads of --impl ours")
   if a.workload == "c4":   # BASELINE configs[3]: key-hash sharded table, 1B keys over 8 GPUs, dim 128 -- the c2 step
     a.dim, a.resident = 128, 125_000_000
   return a
@@ -241,7 +249,8 @@ def cpu_arm(dim, resident, batch, steps, warmup, threads=0, want_resident=100_00
     # at 100M keys, load 0.745) -- no resize during the run, same as the GPU arm's pre-sized table
     table, kind = O.RefTable(dim, resident, threads=n_thr), "reference"
   else:
-    table, kind, n_thr = O.PortTable(dim, resident), "port", 1
+    table, kind = O.PortTable(dim, resident), "port"
+    n_thr = cores["used"] = 1   # the port is single-threaded
   rng = np.random.default_rng(42)
   cdf = zipf_cdf_np(resident)
   fill = 1 << 20
@@ -352,6 +361,21 @@ def bind_to_gpu_numa(gpu_index):
     return prev
   except Exception:
     return None
+
+
+DUMP_BYTES = 16 << 20   # per output, all ranks together: a run writes at most two outputs, 32 MB in all
+
+
+def dump_rows(out_dir, name, rows, world=1):
+  """--dump-outputs: the rows at a fixed, seeded set of positions of `rows` ([n, dim], what a caller of the timed path
+  received in its last step) as out_dir/<name>.npy in float32, at most DUMP_BYTES // world bytes of rows.  The
+  benchmark's inputs are seeded, so two builds run with the same arguments can be compared output for output."""
+  import torch
+  n, dim = rows.shape
+  keep = max(1, DUMP_BYTES // (4 * dim * world))
+  idx = np.sort(np.random.default_rng(0).choice(n, min(n, keep), replace=False))
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, name + ".npy"), rows[torch.from_numpy(idx).to(rows.device)].float().cpu().numpy())
 
 
 def measured_peak_gbs():
@@ -497,6 +521,10 @@ def gpu_arm(args):
   free = torch.cuda.mem_get_info()[0]
   while 2 * resident * (8 + dim * 4) * 1.1 + (12 << 30) > free and resident > (1 << 20):
     resident //= 2  # smaller GPU than a B200: shrink and say so in config
+  if args.dump_outputs and resident != args.resident:
+    # a smaller table is a different key stream: its outputs cannot be compared with a run at the requested size
+    raise SystemExit("bench.py: %.1f GB free on cuda:%d holds %d resident keys, not the %d asked for; --dump-outputs "
+                     "needs the requested workload" % (free / 1e9, local_rank, resident, args.resident))
   vocab = resident * world
 
   gen = torch.Generator(device=dev).manual_seed(42 + rank)
@@ -595,10 +623,13 @@ def gpu_arm(args):
   barrier()
   t_start.record()
   for s in range(args.steps):
-    step(args.warmup + s, evs[s])
+    out = step(args.warmup + s, evs[s])
   t_end.record()
   barrier()
   clocks = sampler.stop() if rank == 0 else None
+  if args.dump_outputs:
+    dump_rows(args.dump_outputs, "lookup_rows" if world == 1 else "lookup_rows_rank%d" % rank, out.reshape(-1, dim), world)
+  del out
   total_ms = t_start.elapsed_time(t_end)
   find_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in evs]))
   ins_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in evs]))
@@ -859,8 +890,10 @@ def gpu_arm(args):
       table.close()
       del table, var, key_batches, val_batches
       torch.cuda.empty_cache()
-      line["c3"] = c3_measure(args, steps=min(args.steps, 50), warmup=5)
+      line["c3"] = c3_measure(args, steps=args.steps, warmup=5)
     except Exception as ex:
+      if args.dump_outputs:
+        raise   # the c3 output was asked for: no silent gap in the dump
       line["c3"] = {"error": repr(ex)}
   if world == 1 and not args.no_cpu_baseline:
     try:
@@ -968,10 +1001,13 @@ def c3_measure(args, steps, warmup):
   t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
   t0.record()
   for i in range(steps):
-    step(warmup + i)
+    out = step(warmup + i)
   t1.record()
   torch.cuda.synchronize()
   ms = t0.elapsed_time(t1) / steps
+  if args.dump_outputs:
+    dump_rows(args.dump_outputs, "c3_lookup_sparse", out)
+  del out
   # where the step goes: the same step with CUDA events between its phases (outside the timed region)
   phases = {"lookup_sparse": [], "backward_unique_gradsum_apply": []}
   for i in range(5):

@@ -1,7 +1,9 @@
 """oracle/gen_golden.py -- writes tests/golden/*.npz from the REFERENCE engine (oracle/_ref =
-the reference's own libcuckoo compiled from /root/reference).  Run in the authoring container:
-    python oracle/gen_golden.py
-The fixtures are committed; the GPU box (no /root/reference) replays them against the CUDA path
+the reference's own libcuckoo, built by oracle/Makefile when the reference tree is present):
+    python oracle/gen_golden.py [table_ops] [traces]      (both when no argument is given)
+table_ops: tests/golden/table_ops_dim*.npz, op streams with every input and output.
+traces:    tests/golden/ref_engine_traces.npz, digests of what the op streams of tests/helpers.py observe.
+The fixtures are committed; machines without the reference replay them against the CUDA path
 and against the C port.  TEST INFRASTRUCTURE ONLY.
 """
 import os
@@ -11,6 +13,7 @@ import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import oracle as O  # noqa: E402
+from tests import helpers as H  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
@@ -67,15 +70,45 @@ def op_stream(dim, seed, n0=2000, threads=1):
   return g
 
 
-def main():
-  O.build()
-  assert O.have_ref(), "oracle/_ref not built: /root/reference needed to generate goldens"
-  os.makedirs(OUT, exist_ok=True)
+def table_ops():
   for dim, n0 in ((1, 2000), (8, 1000), (16, 1000), (64, 400), (128, 250)):
     g = op_stream(dim, seed=1000 + dim, n0=n0)
     path = os.path.join(OUT, "table_ops_dim%d.npz" % dim)
     np.savez_compressed(path, **g)
     print(path, os.path.getsize(path) >> 10, "KiB", "final size", int(g["size3"]))
+
+
+def _trace(stream, *args):
+  rec = H.Trace()
+  stream(*args, rec)
+  return rec.array()
+
+
+def traces():
+  g = {}
+  for dim in (1, 16, 64, 128):
+    g["random_ops_dim%d" % dim] = _trace(H.stream_random_ops, O.RefTable(dim, 0, threads=1), dim)
+  # the sharded launchers (cuckoo_hashtable_op.cc:39-182) over 4 threads give the same set as 1 thread
+  g["set_semantics"] = _trace(H.stream_set_semantics, O.RefTable(16, 0, threads=4))
+  assert np.array_equal(g["set_semantics"], _trace(H.stream_set_semantics, O.RefTable(16, 0, threads=1)))
+  for c, (dim, init_size, ops) in enumerate(H.small_op_streams()):
+    g["small_ops_%d" % c] = _trace(H.stream_small_ops, O.RefTable(dim, init_size, threads=1), dim, ops)
+  np.savez_compressed(H.TRACES, **g)
+  print(H.TRACES, os.path.getsize(H.TRACES) >> 10, "KiB", sum(v.shape[0] for v in g.values()), "digests")
+
+
+def main():
+  what = sys.argv[1:] or ["table_ops", "traces"]
+  unknown = set(what) - {"table_ops", "traces"}
+  if unknown:
+    sys.exit("gen_golden.py: unknown fixture set(s) %s; expected table_ops and/or traces" % ", ".join(sorted(unknown)))
+  O.build()
+  assert O.have_ref(), "oracle/_ref not built: the reference tree is needed to generate goldens"
+  os.makedirs(OUT, exist_ok=True)
+  if "table_ops" in what:
+    table_ops()
+  if "traces" in what:
+    traces()
 
 
 if __name__ == "__main__":

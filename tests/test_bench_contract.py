@@ -37,6 +37,31 @@ def test_other_ranks_of_the_reference_arm_exit_quietly():
   assert p.returncode == 0 and p.stdout.strip() == ""
 
 
+def test_dump_outputs_writes_the_same_float32_sample_every_time(tmp_path):
+  sys.path.insert(0, ROOT)
+  import bench as B
+  import torch
+  dim = 256
+  keep = B.DUMP_BYTES // (4 * dim)
+  rows = torch.randn(3 * keep, dim, generator=torch.Generator().manual_seed(0))
+  rows[:, 0] = torch.arange(rows.shape[0])                             # column 0 = the row's position
+  B.dump_rows(str(tmp_path / "a"), "rows", rows)
+  B.dump_rows(str(tmp_path / "b"), "rows", rows.clone())
+  a, b = np.load(tmp_path / "a" / "rows.npy"), np.load(tmp_path / "b" / "rows.npy")
+  assert a.dtype == np.float32 and a.shape == (keep, dim) and a.nbytes <= B.DUMP_BYTES
+  np.testing.assert_array_equal(a, b)                                  # the same positions in every run
+  pos = a[:, 0].astype(np.int64)
+  assert np.unique(pos).shape[0] == pos.shape[0]
+  np.testing.assert_array_equal(a, rows.numpy()[pos])                  # every dumped row is a row of the output
+  B.dump_rows(str(tmp_path / "c"), "rows", rows, world=4)
+  assert np.load(tmp_path / "c" / "rows.npy").shape == (keep // 4, dim)   # the ranks share the budget
+  B.dump_rows(str(tmp_path / "d"), "rows", rows[:, :1].repeat(1, 2 * dim))   # wider rows: fewer of them, same bytes
+  assert np.load(tmp_path / "d" / "rows.npy").nbytes <= B.DUMP_BYTES
+  p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--dump-outputs", str(tmp_path)],
+                     capture_output=True, text=True, timeout=120, cwd=ROOT)
+  assert p.returncode != 0 and "--dump-outputs" in p.stderr              # never a silent run without the dump
+
+
 def test_zipf_key_stream_helpers():
   sys.path.insert(0, ROOT)
   import bench as B

@@ -1,9 +1,11 @@
-"""CPU tests of the oracle itself: the C port and (when built here) the reference's own libcuckoo against
-the reference's known-answer tests and against each other.  No GPU."""
+"""CPU tests of the oracle itself: the C port (and the reference's own libcuckoo, when built here) against the
+reference's known-answer tests, and the port against what the reference engine computed on the same op streams
+(tests/golden/ref_engine_traces.npz).  No GPU."""
 import numpy as np
 import pytest
 
 from oracle import oracle as O
+from tests import helpers as H
 from tests.helpers import golden_files, replay_golden
 
 ENGINES = ["port"] + (["ref"] if O.have_ref() else [])
@@ -57,56 +59,24 @@ def test_golden_streams(engine, path):
   replay_golden(make(engine, int(g["dim"])), g)
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built (no /root/reference)")
 @pytest.mark.parametrize("dim", [1, 16, 64, 128])
 def test_port_equals_reference_engine(dim):
-  """Same random op stream into the port and the reference's libcuckoo: identical results INCLUDING
-  export (iteration) order, through several doublings and cuckoo displacements."""
-  r, p = O.RefTable(dim, 0, threads=1), O.PortTable(dim, 0)
-  rng = np.random.default_rng(dim)
-  for it in range(24):
-    n = int(rng.integers(1, 4000))
-    keys = rng.integers(0, 15000, size=n).astype(np.int64)
-    op = it % 4
-    if op == 0:
-      v = rng.standard_normal((n, dim)).astype(np.float32)
-      r.insert(keys, v), p.insert(keys, v)
-    elif op == 1:
-      d = rng.standard_normal((n, dim)).astype(np.float32)
-      a, ea = r.find(keys, d, True)
-      b, eb = p.find(keys, d, True)
-      np.testing.assert_array_equal(a, b)
-      np.testing.assert_array_equal(ea, eb)
-    elif op == 2:
-      ex = rng.integers(0, 2, size=n).astype(bool)
-      v = rng.standard_normal((n, dim)).astype(np.float32)
-      r.accum(keys, v, ex), p.accum(keys, v, ex)
-    else:
-      r.remove(keys[:n // 4]), p.remove(keys[:n // 4])
-    assert r.size() == p.size()
-    ka, va = r.export()
-    kb, vb = p.export()
-    np.testing.assert_array_equal(ka, kb)
-    np.testing.assert_array_equal(va, vb)
+  """Same random op stream into the port as into the reference's libcuckoo (recorded; replayed on it too when it is
+  built here): identical results INCLUDING export (iteration) order, through several doublings and cuckoo displacements."""
+  for engine in ENGINES:
+    rec = H.Trace()
+    H.stream_random_ops(make(engine, dim), dim, rec)
+    H.assert_trace("random_ops_dim%d" % dim, rec, engine)
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built")
 def test_reference_engine_multithreaded_set_semantics():
-  """The sharded launchers (cuckoo_hashtable_op.cc:39-182) over 4 threads give the same SET as 1 thread."""
-  dim = 16
-  a, b = O.RefTable(dim, 0, threads=4), O.RefTable(dim, 0, threads=1)
-  rng = np.random.default_rng(7)
-  keys = rng.permutation(200000)[:100000].astype(np.int64)
-  vals = rng.standard_normal((keys.shape[0], dim)).astype(np.float32)
-  a.insert(keys, vals), b.insert(keys, vals)
-  q = rng.integers(0, 200000, 50000).astype(np.int64)
-  d = np.zeros(dim, np.float32)
-  np.testing.assert_array_equal(a.find(q, d), b.find(q, d))
-  ka, va = a.export()
-  kb, vb = b.export()
-  oa, ob = np.argsort(ka), np.argsort(kb)
-  np.testing.assert_array_equal(ka[oa], kb[ob])
-  np.testing.assert_array_equal(va[oa], vb[ob])
+  """The sharded launchers (cuckoo_hashtable_op.cc:39-182) of the reference engine over 4 threads give the same find
+  results and the same SET as one thread: the recorded one-thread result, which the reference engine over 4 threads
+  (when it is built here) and the single-threaded port must both reproduce."""
+  for engine in ENGINES:
+    rec = H.Trace()
+    H.stream_set_semantics(make(engine, 16, 0, threads=4), rec)
+    H.assert_trace("set_semantics", rec, engine)
 
 
 def test_default_partition_fn():
@@ -187,53 +157,19 @@ def test_twin_adagrad_matches_dense():
   np.testing.assert_array_equal(v[np.argsort(k)], dense_p[np.sort(k)])
 
 
-# ---- property-based pinning of the C port against the reference's own engine -----------------------------
-try:
-  from hypothesis import given, settings, strategies as st
-  _HAVE_HYP = True
-except Exception:  # pragma: no cover
-  _HAVE_HYP = False
-
-if _HAVE_HYP:
-  _op = st.tuples(st.sampled_from(["insert", "accum", "remove", "find", "clear"]),
-                  st.lists(st.integers(min_value=-40, max_value=40), min_size=0, max_size=60),
-                  st.integers(min_value=0, max_value=2**31 - 1))
-
-  @pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref not built")
-  @settings(max_examples=60, deadline=None)
-  @given(st.sampled_from([1, 3, 16]), st.sampled_from([1, 4, 64]), st.lists(_op, min_size=1, max_size=25))
-  def test_port_vs_reference_engine_property(dim, init_size, ops):
-    """Arbitrary op streams over a tiny key universe and tiny initial tables (init_size 1/4/64 slots: every
-    insert path runs -- last-empty-slot placement, BFS displacement, doubling): the C port and the reference's
-    libcuckoo agree on sizes, find results, exists masks and export ORDER after every op.  Duplicate keys inside a
-    call are allowed here (both engines are single-threaded, so the outcome is deterministic)."""
-    r, p = O.RefTable(dim, init_size, threads=1), O.PortTable(dim, init_size)
-    for name, keys, seed in ops:
-      k = np.array(keys, dtype=np.int64)
-      rng = np.random.default_rng(seed)
-      if name == "insert":
-        v = rng.integers(-5, 5, size=(k.shape[0], dim)).astype(np.float32)
-        r.insert(k, v), p.insert(k, v)
-      elif name == "accum":
-        v = rng.integers(-5, 5, size=(k.shape[0], dim)).astype(np.float32)
-        ex = rng.integers(0, 2, size=k.shape[0]).astype(bool)
-        r.accum(k, v, ex), p.accum(k, v, ex)
-      elif name == "remove":
-        r.remove(k), p.remove(k)
-      elif name == "clear":
-        r.clear(), p.clear()
-      else:
-        d = rng.integers(-9, 9, size=(max(1, k.shape[0]), dim)).astype(np.float32)
-        a, ea = r.find(k, d if k.shape[0] else d[0], True)
-        b, eb = p.find(k, d if k.shape[0] else d[0], True)
-        np.testing.assert_array_equal(ea, eb)
-        np.testing.assert_array_equal(a, b)
-      assert r.size() == p.size()
-      ka, va = r.export()
-      kb, vb = p.export()
-      np.testing.assert_array_equal(ka, kb)
-      np.testing.assert_array_equal(va, vb)
-    r.close(), p.close()
+# ---- pinning of the C port against the reference's own engine on many small op streams ---------------------------
+def test_port_vs_reference_engine_property():
+  """60 seeded op streams over a tiny key universe and tiny initial tables (init_size 1/4/64 slots: every insert path
+  runs -- last-empty-slot placement, BFS displacement, doubling): the C port and the reference's libcuckoo (recorded;
+  replayed on it too when it is built here) agree on sizes, find results, exists masks and export ORDER after every op.
+  Duplicate keys inside a call are allowed here (both engines are single-threaded, so the outcome is deterministic)."""
+  for engine in ENGINES:
+    for c, (dim, init_size, ops) in enumerate(H.small_op_streams()):
+      rec = H.Trace()
+      t = make(engine, dim, init_size)
+      H.stream_small_ops(t, dim, ops, rec)
+      t.close()
+      H.assert_trace("small_ops_%d" % c, rec, engine)
 
 
 def test_optimizer_rules_against_an_independent_implementation():
